@@ -15,9 +15,9 @@ replicated result of the LAST timed step is checked on rank 0 against the CPU po
 reference (<= 1e-6 relative) at every N.
 
 value      whole-job GEdge/s, inputs resident in HBM, CUDA events on the library's stream, max over ranks.
-e2e        the same call made the way a user of the reference makes it -- the UNMODIFIED pygraphblas.Matrix.mxv
-           (baseline/_ref, staged from /root/reference) over suitesparse_graphblas/ -> libb200grb.so -- with u coming
-           from pinned host memory and w (values + presence) going back to pinned host memory inside the timed region.
+e2e        the same call made the way a user of the reference makes it -- Matrix.mxv of the host-side mirror of the
+           reference's interface -> libb200grb.so -- with u coming from pinned host memory and w (values + presence)
+           going back to pinned host memory inside the timed region.
 roofline   algorithmic bytes of one local SpMV / device time of one step of the SAME timed loop; the dominant kernel's
            share of the step comes from the committed ncu launch list (profiles/).
 The line also carries SpGEMM (configs[3]) with its own roofline and CPU baseline, BFS (configs[2]) and SSSP (configs[4]
@@ -200,6 +200,23 @@ def P(a):
     return a.ctypes.data_as(ctypes.c_void_p)
 
 
+DUMP_BYTES = 64_000_000
+
+
+def dump_outputs(dirname, x, present):
+    """--dump-outputs DIR: the result vector w of the last timed step, as a caller of mxv receives it, in DIR/<name>.npy:
+    w_values (float32, 0 where w has no entry) and w_present (float32, 1 where it has one).  Above DUMP_BYTES in all, a
+    fixed seeded sample of the rows is written instead, with their ids in w_rows (float64)."""
+    out = {"w_values": np.where(present != 0, x, 0).astype(np.float32), "w_present": (present != 0).astype(np.float32)}
+    if 8 * len(x) > DUMP_BYTES - 4096:
+        rows = np.sort(np.random.default_rng(0).choice(len(x), size=(DUMP_BYTES - 4096) // 16, replace=False))
+        out = {k: v[rows] for k, v in out.items()}
+        out["w_rows"] = rows.astype(np.float64)
+    os.makedirs(dirname, exist_ok=True)
+    for name, a in out.items():
+        np.save(os.path.join(dirname, name + ".npy"), a)
+
+
 def cpu_spmv(n, indptr, indices, vals, u, min_seconds, max_reps):
     """The OpenMP port in its best measured configuration; returns (threads_used, budget, times, w, presence)."""
     L = oracle_lib()
@@ -249,8 +266,10 @@ def run_reference(args):
     nnz = len(indices)
     vals, u = spmv_inputs(nnz, n)
     cpu_spmv(n, indptr, indices, vals, u, 0.0, max(args.warmup, 1))
-    threads, info, times, _, _ = cpu_spmv(n, indptr, indices, vals, u, float("inf"), args.steps)      # exactly K timed passes
+    threads, info, times, w, pres = cpu_spmv(n, indptr, indices, vals, u, float("inf"), args.steps)      # exactly K timed passes
     times = times[:args.steps]
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, w, pres)
     ms = 1e3 * float(np.median(times))
     value = nnz / (ms * 1e-3) / 1e9
     sample = f"{len(times)} full SpMV passes over the scale-{args.scale} graph ({nnz} edges each), median"
@@ -338,6 +357,11 @@ def run_b200(args):
     sync_all()
     launches = lib.B200_kernel_launches() - launches0
     ms_total = e0.elapsed_time(e1)
+    if args.dump_outputs:
+        # read back before the loops below run the same mxv again
+        x_last, p_last = comm.allgather(w, r0).to_numpy() if comm is not None else w.to_numpy()
+        if rank == 0:
+            dump_outputs(args.dump_outputs, x_last if newid is None else x_last[newid], p_last if newid is None else p_last[newid])
     local_ms = ms_total / args.steps
     if world > 1:
         # the exchange's share of a step: a second pass of the same loop with events around each local SpMV (kept out of the
@@ -418,7 +442,7 @@ def run_b200(args):
         out["parity_what"] = ("replicated result of the last timed step on rank 0: presence bit pattern == non-empty rows (and == the CPU port's), "
                               "values <= 1e-6 relative vs an fp64 scipy reference (N = 1 also: presence == the CPU port's, values within 2e-5 of its fp32 row-order sums)")
 
-    # ---- end to end with host buffers through the reference's own API (N = 1: the call a pygraphblas user makes)
+    # ---- end to end with host buffers through the mirror of the reference's API (the call a pygraphblas user makes)
     out["e2e"] = bench_e2e(ctx, A, ncols_l, lrows, nnz, u_host if world == 1 else u.to_numpy()[0], x_rep if world == 1 else None)
 
     if rank == 0 and world == 1:
@@ -457,9 +481,8 @@ def run_b200(args):
 
 def bench_e2e(ctx, A_mirror, n, lrows, nnz, u_host, x_dev):
     """One step = u (pinned host) -> HBM, Matrix.mxv, w values + presence -> pinned host; A stays resident in HBM as it
-    stays in the reference's process memory.  At N = 1 the mxv is the reference's OWN pygraphblas.Matrix.mxv
-    (/root/reference/pygraphblas/matrix.py:2586-2726, staged unmodified in baseline/_ref) over the binding stub; the bulk
-    dense import/export entry points stand in for the per-element setElement loop the reference would otherwise use."""
+    stays in the reference's process memory.  The mxv is the mirror's Matrix.mxv (the reference's matrix.py:2586-2726);
+    the bulk dense import/export entry points stand in for the per-element setElement loop the reference would otherwise use."""
     torch, gb, args, world, rank = ctx["torch"], ctx["gb"], ctx["args"], ctx["world"], ctx["rank"]
     lib, ffi = gb.lib, gb.ffi
     from pygraphblas_b200 import Vector, FP32
@@ -473,31 +496,6 @@ def bench_e2e(ctx, A_mirror, n, lrows, nnz, u_host, x_dev):
     we = [Vector.sparse(FP32, lrows) for _ in range(NB)]
     through = "pygraphblas_b200.Matrix.mxv (host-side mirror of the reference's method)"
     mxv = lambda b: A_mirror.mxv(ue[b], semiring=FP32.PLUS_TIMES, out=we[b])
-    staged = os.path.join(ROOT, "baseline", "_ref")
-    keep = []
-    if world == 1 and os.path.isdir(os.path.join(staged, "pygraphblas")):
-        try:
-            if staged not in sys.path:
-                sys.path.insert(1, staged)
-            import pygraphblas as ref                           # the UNMODIFIED reference package, on the binding stub
-            assert os.path.realpath(ref.__file__).startswith(os.path.realpath(staged))
-            # the reference wraps raw handles (matrix.py:99-107); give it handles of its own
-            hA = ffi.new("GrB_Matrix*")
-            assert lib.GrB_Matrix_dup(hA, A_mirror._matrix[0]) == 0
-            rA = ref.Matrix(hA)
-            assert rA.type is ref.FP32 and rA.nvals == nnz
-            ru, rw = [], []
-            for b in range(NB):
-                hu, hw = ffi.new("GrB_Vector*"), ffi.new("GrB_Vector*")
-                assert lib.GrB_Vector_dup(hu, ue[b]._vector[0]) == 0 and lib.GrB_Vector_new(hw, lib.GrB_FP32, lrows) == 0
-                ru.append(ref.Vector(hu)); rw.append(ref.Vector(hw))
-            rsr = ref.FP32.PLUS_TIMES
-            keep = [ue, we]
-            ue, we = ru, rw                                      # the copies below act on the reference's handles
-            mxv = lambda b: rA.mxv(ru[b], semiring=rsr, out=rw[b])
-            through = "pygraphblas.Matrix.mxv of the UNMODIFIED reference (baseline/_ref) -> suitesparse_graphblas stub -> GrB_mxv"
-        except Exception as e:
-            through += f" [reference import failed: {type(e).__name__}: {e}]"[:200]
     up = [ffi.cast("void*", x.ctypes.data) for x in u_pin]
     wp = [ffi.cast("void*", x.ctypes.data) for x in w_pin]
     pp = [ffi.cast("uint8_t*", x.ctypes.data) for x in p_pin]
@@ -560,7 +558,6 @@ def bench_e2e(ctx, A_mirror, n, lrows, nnz, u_host, x_dev):
         res["mismatch"] = diag
     if x_dev is not None:
         res["matches_device_result"] = bool(same and np.array_equal(w_serial[p_serial != 0], x_dev[p_serial != 0]))
-    del keep
     return res
 
 
@@ -1096,7 +1093,10 @@ def main():
     ap.add_argument("--no-extras", "--no-spgemm", dest="no_extras", action="store_true")
     ap.add_argument("--cpu-seconds", type=float, default=10.0)
     ap.add_argument("--quick", action="store_true", help="timed SpMV loop only (for ncu): no e2e / CPU baseline / extras")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the result of the last timed step to DIR/*.npy (float32)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.impl == "reference":
         run_reference(args)
     else:

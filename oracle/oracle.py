@@ -47,11 +47,20 @@ CMP_OPS = {"EQ", "NE", "GT", "LT", "GE", "LE"}
 
 
 def build(force=False):
+    global _BUILD, _LIB
     srcs = [s for s in _SOURCES if os.path.exists(s)]
     if (not force and os.path.exists(_LIB)
             and all(os.path.getmtime(_LIB) >= os.path.getmtime(s) for s in srcs)):
         return _LIB
-    os.makedirs(_BUILD, exist_ok=True)
+    try:
+        os.makedirs(_BUILD, exist_ok=True)
+        writable = os.access(_BUILD, os.W_OK)
+    except OSError:
+        writable = False
+    if not writable:                 # a read-only checkout: build per process in a temporary directory
+        import tempfile
+        _BUILD = tempfile.mkdtemp(prefix="b200grb_oracle_")
+        _LIB = os.path.join(_BUILD, "liboracle.so")
     cmd = ["gcc", "-O3", "-march=native", "-fopenmp", "-fPIC", "-shared", "-std=gnu11", "-o", _LIB] + srcs + ["-lm"]
     r = subprocess.run(cmd, capture_output=True, text=True)
     if r.returncode != 0:

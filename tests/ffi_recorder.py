@@ -1,9 +1,9 @@
-"""Side-by-side recorder for the host-side mirror (used by tests/test_reference_dropin.py in a subprocess, CPU
-container only: it needs /root/reference).  The library's compute entry points are replaced by a recorder BEFORE
-the reference package and the mirror are imported, so both packages capture the same objects; every call is
-normalised at record time (operator handle -> name, descriptor -> field values, vector / matrix -> type, shape,
-nvals, index list -> its values) and nothing computes.  `both(fn)` returns what the reference and the mirror
-pass to the C ABI for the same user-level expression."""
+"""Recorder of the C calls a GraphBLAS package makes (used by tests/test_reference_dropin.py and
+tests/golden/make_dropin_goldens.py, each in a subprocess of its own).  The library's compute entry points are
+replaced by a recorder BEFORE the package under test (the mirror, or the reference over the binding stub) is
+imported, so it captures the recorder; every call is normalised at record time (operator handle -> name, descriptor
+-> field values, vector / matrix -> type, shape, nvals, index list -> its values) and nothing computes.
+`run(fn, pkg)` returns what `pkg` passes to the C ABI for the user-level expression `fn(pkg)`."""
 import os
 import importlib.util, sys
 _spec = importlib.util.spec_from_file_location("pygraphblas_b200._ffi", os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file__))), "pygraphblas_b200", "_ffi.py"))
@@ -31,7 +31,6 @@ class Recorder:
 
 _ffi.lib = Recorder()
 import pygraphblas_b200 as gb          # noqa: E402
-import pygraphblas as ref              # noqa: E402
 ffi = gb.ffi
 KIND = {"struct GB_BinaryOp_opaque *": 0, "struct GB_Monoid_opaque *": 1, "struct GB_Semiring_opaque *": 2, "struct GB_UnaryOp_opaque *": 3}
 
@@ -119,7 +118,3 @@ def run(fn, pkg):
     except Exception as e:
         return ("EXC", type(e).__name__, str(e)[:60])
     return tuple(CALLS[n0:])
-
-
-def both(fn):
-    return run(fn, ref), run(fn, gb)

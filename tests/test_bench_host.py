@@ -53,3 +53,22 @@ def test_streamed_sample_is_a_row_subset_of_the_parent():
 def test_both_arms_share_one_workload_dict():
     a = bench.workload_config(22, 1 << 22, 65242949)
     assert a == bench.workload_config(22, 1 << 22, 65242949) and "workload" in a and "model" not in a
+
+
+def test_dump_outputs_writes_the_result_vector_within_the_size_limit(tmp_path):
+    rng = np.random.default_rng(1)
+    x, present = rng.random(1000, dtype=np.float32), (rng.random(1000) < 0.5).astype(np.uint8)
+    bench.dump_outputs(str(tmp_path / "full"), x, present)
+    w, p = np.load(tmp_path / "full" / "w_values.npy"), np.load(tmp_path / "full" / "w_present.npy")
+    assert w.dtype == p.dtype == np.float32 and not os.path.exists(tmp_path / "full" / "w_rows.npy")
+    assert np.array_equal(p, present.astype(np.float32)) and np.array_equal(w, np.where(present != 0, x, 0))
+    # above the limit: the same seeded sample of rows every time
+    n = bench.DUMP_BYTES // 8 + 1000
+    x, present = np.arange(n, dtype=np.float32), np.ones(n, np.uint8)
+    for d in ("a", "b"):
+        bench.dump_outputs(str(tmp_path / d), x, present)
+    sizes = sum(os.path.getsize(tmp_path / "a" / f) for f in os.listdir(tmp_path / "a"))
+    assert sizes <= bench.DUMP_BYTES
+    rows = np.load(tmp_path / "a" / "w_rows.npy")
+    assert rows.dtype == np.float64 and np.array_equal(rows, np.load(tmp_path / "b" / "w_rows.npy"))
+    assert np.array_equal(np.load(tmp_path / "a" / "w_values.npy"), rows.astype(np.float32))
