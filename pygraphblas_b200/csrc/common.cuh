@@ -57,6 +57,7 @@ enum UnaryCode : int {
     UOP_COUNT
 };
 
+struct RunFix;
 // Device CSR panel: rows sorted, columns sorted inside each row.
 struct Csr {
     int64_t nrows = 0, ncols = 0, nnz = 0;
@@ -72,8 +73,8 @@ struct Csr {
     uint32_t *run_headw = nullptr;   // [ceil(nnz/32)] bit q = entry q starts a row
     uint16_t *run_lane = nullptr;    // [nruns*32] row starts inside the run before the lane's first entry
     uint32_t *run_base = nullptr;    // [nruns+1] row starts before the run (= rank of its first row start)
-    int32_t *run_tail_row = nullptr; // [nruns] row still open at the end of the run (its last row start), or -1
-    uint32_t *run_tail_last = nullptr; // [nruns] last run that row reaches
+    RunFix *run_fix = nullptr;       // [run_fix_long + run_fix_short] fix-up items (spmv_args.cuh), the long ones first
+    int64_t run_fix_long = 0, run_fix_short = 0;
     uint32_t *nzrow = nullptr;       // [nnzrows] ids of the non-empty rows, ascending
     uint8_t *pres_tmpl = nullptr;    // [nrows] 1 where the row is non-empty
     int64_t nruns = 0, nnzrows = 0;

@@ -193,8 +193,8 @@ GrB_Info ws_get(int slot, void **p, size_t bytes, std::string *err, bool *fresh)
 void csr_drop_plans(Csr &c) {
     dfree(c.tile_row); c.tile_row = nullptr; c.ntiles = 0; c.tile_size = 0;
     dfree(c.hperm); dfree(c.hcol); c.hperm = nullptr; c.hcol = nullptr; c.henc = 0; c.hot_planned = false; c.hot_cover = 0.0;
-    dfree(c.run_headw); dfree(c.run_lane); dfree(c.run_base); dfree(c.run_tail_row); dfree(c.run_tail_last); dfree(c.nzrow); dfree(c.pres_tmpl);
-    c.run_headw = nullptr; c.run_lane = nullptr; c.run_base = nullptr; c.run_tail_row = nullptr; c.run_tail_last = nullptr; c.nzrow = nullptr; c.pres_tmpl = nullptr;
+    dfree(c.run_headw); dfree(c.run_lane); dfree(c.run_base); dfree(c.run_fix); dfree(c.nzrow); dfree(c.pres_tmpl);
+    c.run_headw = nullptr; c.run_lane = nullptr; c.run_base = nullptr; c.run_fix = nullptr; c.run_fix_long = c.run_fix_short = 0; c.nzrow = nullptr; c.pres_tmpl = nullptr;
     c.nruns = 0; c.nnzrows = 0;
     dfree(c.ws_head); dfree(c.ws_tail); dfree(c.ws_head_has); dfree(c.ws_tail_has); dfree(c.ws_uhot);
     c.ws_head = c.ws_tail = c.ws_uhot = nullptr; c.ws_head_has = c.ws_tail_has = nullptr;

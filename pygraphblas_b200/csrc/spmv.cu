@@ -472,7 +472,7 @@ static GrB_Info mxv_core(GrB_Vector w, const GrB_Vector mask, const GrB_BinaryOp
         RunArgs ra{};
         ra.col = c.col; ra.aval = aval; ra.uval = uval; ra.headw = c.run_headw; ra.lane_rank = c.run_lane; ra.run_base = c.run_base;
         ra.nzrow = c.nzrow; ra.rowptr = c.rowptr32; ra.nruns = c.nruns; ra.nnz = c.nnz; ra.tval = tval;
-        ra.tail_row = c.run_tail_row; ra.tail_last = c.run_tail_last;
+        ra.fix = c.run_fix; ra.fix_long = c.run_fix_long; ra.fix_short = c.run_fix_short;
         ra.add_op = add; ra.mul_op = kmul; ra.flip = kflip;
         ra.head_val = c.ws_head; ra.tail_val = c.ws_tail;            // scratch kept with the plan (the library serialises calls)
         if (sparse_u) { ra.upres = u->dpres; ra.tpres = tpres; ra.head_has = c.ws_head_has; ra.tail_has = c.ws_tail_has; }
@@ -485,9 +485,10 @@ static GrB_Info mxv_core(GrB_Vector w, const GrB_Vector mask, const GrB_BinaryOp
         } else hot_kb = 0;
         Hot2Args hot{};
         if (hot_kb > 0) {
-            // one launch: u at the hot columns, T cleared, T's presence from the plan
-            spmv_hot2_prep(c, uval, tc_size(xt), tval, (size_t)n * zsz, tpres);
+            // u at the hot columns; the kernel writes T's presence and the values of the empty rows itself
+            spmv_hot2_prep(c, uval, tc_size(xt));
             ra.col = c.hcol; hot.u_hot = c.ws_uhot; hot.henc = c.henc; hot.tab_n = 0;
+            hot.pres_tmpl = c.pres_tmpl; hot.tpres = tpres; hot.nrows = n;
             kernel_name = "run+hot-table (TMA-staged)";
         } else {
             CU_TRY(cudaMemsetAsync(tval, 0, (size_t)n * zsz, G.stream), err);

@@ -3,10 +3,14 @@
 #include "spmv_common.cuh"
 
 static constexpr int RUN = 256;
+// fix-up work item of the run plan: a run that contains a row start, the row still open at its end (its last row start)
+// and the last run that row reaches; 16 bytes, so one load gives a thread all three
+struct __align__(16) RunFix { uint32_t run, row, last, pad; };
+constexpr uint32_t FIX_LANES = 8;             // rows reaching more than this many runs further are folded by 8 lanes, the others by one thread
 struct RunArgs {
     const uint32_t *col; const void *aval; const void *uval;
     const uint32_t *headw; const uint16_t *lane_rank; const uint32_t *run_base; const uint32_t *nzrow; const uint32_t *rowptr;
-    const int32_t *tail_row; const uint32_t *tail_last;       // structural: which row is open at a run's end, how far it reaches
+    const RunFix *fix; int64_t fix_long, fix_short;          // fix-up list: the fix_long items that reach > FIX_LANES runs first
     int64_t nruns; int64_t nnz;
     void *tval;
     void *head_val; void *tail_val;                            // per run: partial of the row it starts inside / of the row open at its end
@@ -20,6 +24,9 @@ struct Hot2Args {
     const void *u_hot;        // [henc] u at the hottest columns (prep kernel)
     uint32_t henc;            // ids below this are hot ranks
     uint32_t tab_n;           // entries of u_hot kept in shared memory (<= henc)
+    const uint8_t *pres_tmpl; // [nrows] the plan's presence template: T's presence bytes (u is dense) ...
+    uint8_t *tpres;           // ... copied here by the kernel, which also writes 0 to T's values of the empty rows
+    int64_t nrows;
 };
 
 // ------------------------------------------------------------------ masked pull with early exit (BFS-shaped calls)

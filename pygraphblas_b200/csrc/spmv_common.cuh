@@ -77,7 +77,7 @@ struct RunArgs;
 GrB_Info spmv_run_plan(Csr &c, std::string *err);
 GrB_Info spmv_hot_plan(Csr &c, std::string *err);
 struct Hot2Args;
-void spmv_hot2_prep(const Csr &c, const void *u, int vsize, void *tval, size_t tval_bytes, uint8_t *tpres);
+void spmv_hot2_prep(const Csr &c, const void *u, int vsize);
 bool spmv_run_dispatch(int xt, int add, int mul, const RunArgs &a, const Hot2Args *hot, size_t table_limit);
 bool spmv_run_generic(int xt, int zt, const RunArgs &a);
 

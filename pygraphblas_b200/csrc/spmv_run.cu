@@ -30,18 +30,30 @@ __global__ void plan_runs_kernel(const uint32_t *headw, int64_t nruns, int64_t n
 __global__ void plan_base_kernel(const int64_t *scan, int64_t nruns, uint32_t *run_base) {
     for (int64_t k = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; k <= nruns; k += (int64_t)gridDim.x * blockDim.x) run_base[k] = (uint32_t)scan[k];
 }
-// the row that starts last inside a run always holds the run's last entry: it is the run's "open" row
-// (possibly ending exactly at the run's end), completed by the fix-up kernel
-__global__ void plan_tails_kernel(const uint32_t *run_base, const uint32_t *nzrow, const uint32_t *rowptr, int64_t nruns,
-                                  int32_t *tail_row, uint32_t *tail_last) {
+// the row that starts last inside a run always holds the run's last entry: it is the run's "open" row (possibly ending
+// exactly at the run's end), completed by the fix-up kernel.  One fix-up item per run that holds a row start.
+__device__ __forceinline__ bool plan_fix_item(const uint32_t *run_base, const uint32_t *nzrow, const uint32_t *rowptr, int64_t k, RunFix &f) {
+    if (run_base[k + 1] == run_base[k]) return false;
+    const uint32_t r = nzrow[run_base[k + 1] - 1];
+    f = RunFix{(uint32_t)k, r, (rowptr[r + 1] - 1) / RUN, 0u};
+    return true;
+}
+// is_long[k] / is_short[k]: run k has an item whose row reaches more / at most FIX_LANES runs further
+__global__ void plan_fix_count_kernel(const uint32_t *run_base, const uint32_t *nzrow, const uint32_t *rowptr, int64_t nruns,
+                                      int64_t *is_long, int64_t *is_short) {
     for (int64_t k = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; k < nruns; k += (int64_t)gridDim.x * blockDim.x) {
-        int32_t tr = -1; uint32_t tl = 0;
-        if (run_base[k + 1] > run_base[k]) {
-            const uint32_t r = nzrow[run_base[k + 1] - 1];
-            const uint32_t re = rowptr[r + 1];
-            tr = (int32_t)r; tl = (re - 1) / RUN;
-        }
-        tail_row[k] = tr; tail_last[k] = tl;
+        RunFix f;
+        const bool has = plan_fix_item(run_base, nzrow, rowptr, k, f);
+        const bool lg = has && f.last - f.run > FIX_LANES;
+        is_long[k] = lg; is_short[k] = has && !lg;
+    }
+}
+// the list in run order, the long items first (their exclusive scans give the slots)
+__global__ void plan_fix_list_kernel(const uint32_t *run_base, const uint32_t *nzrow, const uint32_t *rowptr, int64_t nruns,
+                                     const int64_t *long_at, const int64_t *short_at, int64_t nlong, RunFix *list) {
+    for (int64_t k = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; k < nruns; k += (int64_t)gridDim.x * blockDim.x) {
+        RunFix f;
+        if (plan_fix_item(run_base, nzrow, rowptr, k, f)) list[f.last - f.run > FIX_LANES ? long_at[k] : nlong + short_at[k]] = f;
     }
 }
 static inline int rgrid(int64_t n) { return (int)std::max<int64_t>(1, std::min<int64_t>(ceil_div(n, 256), (int64_t)G.num_sms * 16)); }
@@ -58,8 +70,6 @@ GrB_Info spmv_run_plan(Csr &c, std::string *err) {
     GB_TRY(dalloc(&c.run_headw, (size_t)nwords + 8, err));
     GB_TRY(dalloc(&c.run_lane, (size_t)c.nruns * 32, err));
     GB_TRY(dalloc(&c.run_base, (size_t)c.nruns + 1, err));
-    GB_TRY(dalloc(&c.run_tail_row, (size_t)c.nruns, err));
-    GB_TRY(dalloc(&c.run_tail_last, (size_t)c.nruns, err));
     CU_TRY(cudaMemsetAsync(c.run_headw, 0, ((size_t)nwords + 8) * 4, G.stream), err);
     CU_TRY(cudaMemsetAsync(flag + c.nrows, 0, 8, G.stream), err);
     plan_nonempty_kernel<<<rgrid(c.nrows), 256, 0, G.stream>>>(c.rowptr32, c.nrows, flag, c.pres_tmpl); GB_LAUNCHED();
@@ -74,8 +84,23 @@ GrB_Info spmv_run_plan(Csr &c, std::string *err) {
     plan_runs_kernel<<<(unsigned)ceil_div(c.nruns * 32, 256), 256, 0, G.stream>>>(c.run_headw, c.nruns, nwords, c.run_lane, cnt); GB_LAUNCHED();
     GB_TRY(dev_exclusive_scan(cnt, c.nruns + 1, err));
     plan_base_kernel<<<rgrid(c.nruns + 1), 256, 0, G.stream>>>(cnt, c.nruns, c.run_base); GB_LAUNCHED();
-    plan_tails_kernel<<<rgrid(c.nruns), 256, 0, G.stream>>>(c.run_base, c.nzrow, c.rowptr32, c.nruns, c.run_tail_row, c.run_tail_last); GB_LAUNCHED();
-    dfree(flag); dfree(cnt);
+    // fix-up list: flag the runs by kind into the two halves of `flag2`, scan each, scatter
+    int64_t *flag2 = nullptr;
+    GB_TRY(dalloc(&flag2, 2 * ((size_t)c.nruns + 1), err));
+    int64_t *is_long = flag2, *is_short = flag2 + c.nruns + 1;
+    CU_TRY(cudaMemsetAsync(is_long + c.nruns, 0, 8, G.stream), err);
+    CU_TRY(cudaMemsetAsync(is_short + c.nruns, 0, 8, G.stream), err);
+    plan_fix_count_kernel<<<rgrid(c.nruns), 256, 0, G.stream>>>(c.run_base, c.nzrow, c.rowptr32, c.nruns, is_long, is_short); GB_LAUNCHED();
+    GB_TRY(dev_exclusive_scan(is_long, c.nruns + 1, err));
+    GB_TRY(dev_exclusive_scan(is_short, c.nruns + 1, err));
+    int64_t nfix[2] = {0, 0};
+    CU_TRY(cudaMemcpyAsync(&nfix[0], is_long + c.nruns, 8, cudaMemcpyDeviceToHost, G.stream), err);
+    CU_TRY(cudaMemcpyAsync(&nfix[1], is_short + c.nruns, 8, cudaMemcpyDeviceToHost, G.stream), err);
+    CU_TRY(cudaStreamSynchronize(G.stream), err);
+    c.run_fix_long = nfix[0]; c.run_fix_short = nfix[1];
+    GB_TRY(dalloc(&c.run_fix, (size_t)(nfix[0] + nfix[1]), err));
+    plan_fix_list_kernel<<<rgrid(c.nruns), 256, 0, G.stream>>>(c.run_base, c.nzrow, c.rowptr32, c.nruns, is_long, is_short, nfix[0], c.run_fix); GB_LAUNCHED();
+    dfree(flag); dfree(cnt); dfree(flag2);
     // per-call scratch lives with the plan: partials of the rows that straddle runs (8 bytes covers every type)
     GB_TRY(dmalloc(&c.ws_head, (size_t)c.nruns * 8 + 16, err));
     GB_TRY(dmalloc(&c.ws_tail, (size_t)c.nruns * 8 + 16, err));
@@ -148,29 +173,21 @@ GrB_Info spmv_hot_plan(Csr &c, std::string *err) {
     return GrB_SUCCESS;
 }
 
-// prep for the hot-table kernel, one launch: u_hot[i] = u[hperm[i]] for the henc hottest columns, T's values
-// cleared and its presence bytes set from the plan's template (rows are structurally present or not: u is dense)
-__global__ void __launch_bounds__(256) spmv_hot2_prep_kernel(const uint32_t *hperm, const uint8_t *u, uint8_t *u_hot, int vsize, uint32_t henc,
-                                                            uint4 *tval16, int64_t tval_n16, const uint4 *tmpl16, uint4 *tpres16, int64_t pres_n16) {
-    const int64_t tid = (int64_t)blockIdx.x * blockDim.x + threadIdx.x, nth = (int64_t)gridDim.x * blockDim.x;
-    for (int64_t i = tid; i < henc; i += nth) {
-        const uint32_t col = hperm[i];
-        switch (vsize) {
-            case 1: u_hot[i] = u[col]; break;
-            case 4: ((uint32_t *)u_hot)[i] = ((const uint32_t *)u)[col]; break;
-            default: ((uint64_t *)u_hot)[i] = ((const uint64_t *)u)[col]; break;
-        }
+// prep for the hot-table kernel: u_hot[i] = u[hperm[i]] for the henc hottest columns (the kernel fills T itself)
+__global__ void __launch_bounds__(256) spmv_hot2_prep_kernel(const uint32_t *hperm, const uint8_t *u, uint8_t *u_hot, int vsize, uint32_t henc) {
+    pdl_trigger();                            // the hot-table kernel's prologue needs nothing from here
+    const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= henc) return;
+    const uint32_t col = hperm[i];
+    switch (vsize) {
+        case 1: u_hot[i] = u[col]; break;
+        case 4: ((uint32_t *)u_hot)[i] = ((const uint32_t *)u)[col]; break;
+        default: ((uint64_t *)u_hot)[i] = ((const uint64_t *)u)[col]; break;
     }
-    const uint4 z = make_uint4(0, 0, 0, 0);
-    for (int64_t i = tid; i < tval_n16; i += nth) tval16[i] = z;
-    for (int64_t i = tid; i < pres_n16; i += nth) tpres16[i] = tmpl16[i];
 }
 
-// one launch ahead of the hot-table kernel: u at the hot columns, T cleared, T's presence from the plan's template
-void spmv_hot2_prep(const Csr &c, const void *u, int vsize, void *tval, size_t tval_bytes, uint8_t *tpres) {
-    const int64_t tv16 = (int64_t)((tval_bytes + 15) / 16), pr16 = (c.nrows + 15) / 16;      // buffers are padded by >= 16 bytes
-    spmv_hot2_prep_kernel<<<G.num_sms * 8, 256, 0, G.stream>>>(c.hperm, (const uint8_t *)u, (uint8_t *)c.ws_uhot, vsize, c.henc,
-                                                               (uint4 *)tval, tv16, (const uint4 *)c.pres_tmpl, (uint4 *)tpres, pr16);
+void spmv_hot2_prep(const Csr &c, const void *u, int vsize) {
+    spmv_hot2_prep_kernel<<<(unsigned)ceil_div(c.henc, 256), 256, 0, G.stream>>>(c.hperm, (const uint8_t *)u, (uint8_t *)c.ws_uhot, vsize, c.henc);
     GB_LAUNCHED();
 }
 

@@ -109,7 +109,7 @@ __device__ __forceinline__ void spmv_run_fold(const RunArgs &p, const int64_t ru
     if (lane == 31) { nxt.has = 0; nxt_stop = 0; }
 
     // the lane holding the last row start of the run owns the row that is still open at the run's end
-    // (which row that is, and where it ends, is structural: run_tail_row / run_tail_last of the plan)
+    // (which row that is, and where it ends, is structural: the plan's fix-up list)
     if (seen) {
         const Part<ZT> total = part_join<ZT>(ADD, acc, nxt);
         if (nxt_stop) { const uint32_t row = __ldg(p.nzrow + cur); tval[row] = total.v; if (SPARSE) p.tpres[row] = (uint8_t)total.has; }
@@ -183,6 +183,20 @@ __device__ __forceinline__ void mbar_wait(uint64_t *bar, uint32_t parity) {
                  "@p bra DONE_%=;\n\tbra WAIT_%=;\n\tDONE_%=:\n\t}" ::"r"(smem_u32(bar)), "r"(parity) : "memory");
 }
 
+// Programmatic dependent launch: a kernel launched with launch_pdl may start while the kernel before it on the stream is
+// still running; pdl_wait() returns once that kernel has completed and its writes are visible (a no-op without PDL), and
+// pdl_trigger() lets the next one be launched before this one ends.
+__device__ __forceinline__ void pdl_wait() { asm volatile("griddepcontrol.wait;" ::: "memory"); }
+__device__ __forceinline__ void pdl_trigger() { asm volatile("griddepcontrol.launch_dependents;" ::: "memory"); }
+template <typename... KA, typename... A> static inline void launch_pdl(void (*kernel)(KA...), unsigned grid, unsigned block, size_t smem, A &&...args) {
+    cudaLaunchAttribute attr[1];
+    attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
+    attr[0].val.programmaticStreamSerializationAllowed = 1;
+    cudaLaunchConfig_t cfg{};
+    cfg.gridDim = dim3(grid); cfg.blockDim = dim3(block); cfg.dynamicSmemBytes = smem; cfg.stream = G.stream; cfg.attrs = attr; cfg.numAttrs = 1;
+    cudaLaunchKernelEx(&cfg, kernel, std::forward<A>(args)...);
+}
+
 template <typename XT> __host__ __device__ constexpr int hot2_stage_bytes(bool need_a) { return RUN * 4 + (need_a ? RUN * (int)sizeof(XT) : 0); }
 constexpr int HOT2_WARPS = 32;
 
@@ -216,7 +230,8 @@ __global__ void __launch_bounds__(HOT2_WARPS * 32, 1) spmv_run_hot2_kernel(const
     if (threadIdx.x == 0) mbar_init(s_bar + HOT2_WARPS, 1);
     asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
     __syncthreads();
-    if (threadIdx.x == 0 && h.tab_n) {        // the table: bulk copies of <= 16 KB
+    if (threadIdx.x == 0 && h.tab_n) {        // the table: bulk copies of <= 16 KB of u_hot, once the prep kernel has written it
+        pdl_wait();
         const uint32_t total = h.tab_n * (uint32_t)sizeof(XT);
         mbar_expect_tx(s_bar + HOT2_WARPS, total);
         for (uint32_t off = 0; off < total; off += 16384u)
@@ -224,6 +239,36 @@ __global__ void __launch_bounds__(HOT2_WARPS * 32, 1) spmv_run_hot2_kernel(const
                          min(16384u, total - off), s_bar + HOT2_WARPS);
     }
     if (lane == 0 && run < p.nruns) issue(run);
+
+    // While the table and the first run are in flight: this warp's fixed slice of T's rows gets its presence byte from the
+    // plan's template and, where the row is empty, the value 0.  The non-empty rows are written by spmv_run_fold and the
+    // fix-up only, so these stores never meet theirs and need no ordering.  The 16-byte padding of both arrays is covered
+    // too (presence: template bytes; values: 0), as a 16-byte-granular clear and copy would.
+    {
+        const int64_t rows_p = (h.nrows + 15) & ~(int64_t)15;
+        const int64_t rows_v = ((h.nrows * (int64_t)sizeof(ZT) + 15) & ~(int64_t)15) / (int64_t)sizeof(ZT);
+        const int64_t rows = rows_p > rows_v ? rows_p : rows_v;
+        const int64_t nwarps = (int64_t)gridDim.x * HOT2_WARPS;
+        const int64_t slice = (ceil_div(rows, nwarps) + 31) & ~(int64_t)31;
+        const int64_t r0 = ((int64_t)blockIdx.x * HOT2_WARPS + warp) * slice;
+        const int64_t r1 = r0 + slice < rows ? r0 + slice : rows;
+        ZT *tval = static_cast<ZT *>(p.tval);
+        for (int64_t b = r0; b < r1; b += 4 * 32) {
+            uint8_t t[4];
+#pragma unroll
+            for (int k = 0; k < 4; ++k) { const int64_t r = b + k * 32 + lane; t[k] = r < r1 ? __ldg(h.pres_tmpl + r) : (uint8_t)0; }
+#pragma unroll
+            for (int k = 0; k < 4; ++k) {
+                const int64_t r = b + k * 32 + lane;
+                if (r < r1) {
+                    if (r < rows_p) h.tpres[r] = t[k];
+                    if (r < rows_v && (r >= h.nrows || t[k] == 0)) tval[r] = (ZT)0;
+                }
+            }
+        }
+    }
+    pdl_wait();                               // every thread: the gathers below read u_hot beyond the table
+    pdl_trigger();                            // the fix-up may be launched; it waits for this kernel to complete
     if (h.tab_n) mbar_wait(s_bar + HOT2_WARPS, 0);
 
     const XT *uval = static_cast<const XT *>(p.uval);
@@ -296,29 +341,65 @@ __global__ void __launch_bounds__(HOT2_WARPS * 32, 1) spmv_run_hot2_kernel(const
     }
 }
 
-// rows that continue past their run: tail partial (+) head partials of the following runs, 8 lanes per open row.
-// Every run after `run` up to tail_last starts inside that row, so its head partial exists.
+// The row open at the end of a run: its tail partial (+) the head partials of the following runs up to the last run it
+// reaches (every one of those starts inside the row, so its head partial exists).  One item of the plan's fix-up list each.
+// The association order is fixed whatever the row's length: lane s of 8 folds head[run+1+s], head[run+9+s], ... (lane 0
+// starts with the tail), then lanes combine by the xor butterfly 4, 2, 1.  Items reaching <= FIX_LANES runs have at most one
+// head per lane: one thread evaluates the same tree.  The long items come first in the list and take 8 lanes each.
 template <typename ZT, int ADD_C, bool SPARSE>
 __global__ void __launch_bounds__(256) spmv_run_fixup_kernel(const RunArgs p) {
+    pdl_wait();                               // the partials of the run kernel
     const int ADD = ADD_C >= 0 ? ADD_C : p.add_op;
-    const int sub = threadIdx.x & 7;
-    const int64_t run = ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 3;
-    const int32_t r = run < p.nruns ? __ldg(p.tail_row + run) : -1;
-    Part<ZT> acc{(ZT)0, 0};
-    if (r >= 0) {
-        const int64_t last_run = __ldg(p.tail_last + run);
-        if (sub == 0) { acc.v = static_cast<const ZT *>(p.tail_val)[run]; acc.has = SPARSE ? (int)p.tail_has[run] : 1; }
-        for (int64_t t = run + 1 + sub; t <= last_run; t += 8) {
-            const Part<ZT> y{static_cast<const ZT *>(p.head_val)[t], SPARSE ? (int)p.head_has[t] : 1};
+    const ZT *head = static_cast<const ZT *>(p.head_val);
+    const int64_t long_threads = p.fix_long * FIX_LANES;
+    const int64_t long_ctas = ceil_div(long_threads, 256);
+    if ((int64_t)blockIdx.x < long_ctas) {
+        const int64_t tid = (int64_t)blockIdx.x * 256 + threadIdx.x;
+        const int sub = threadIdx.x & (FIX_LANES - 1);
+        const bool ok = tid < long_threads;
+        RunFix f{0u, 0u, 0u, 0u};
+        if (ok) { const uint4 w = __ldg(reinterpret_cast<const uint4 *>(p.fix + tid / FIX_LANES)); f = RunFix{w.x, w.y, w.z, w.w}; }
+        Part<ZT> acc{(ZT)0, 0};
+        if (ok) {
+            if (sub == 0) { acc.v = static_cast<const ZT *>(p.tail_val)[f.run]; acc.has = SPARSE ? (int)p.tail_has[f.run] : 1; }
+            for (int64_t t = (int64_t)f.run + 1 + sub; t <= (int64_t)f.last; t += FIX_LANES) {
+                const Part<ZT> y{head[t], SPARSE ? (int)p.head_has[t] : 1};
+                acc = part_join<ZT>(ADD, acc, y);
+            }
+        }
+#pragma unroll
+        for (int o = 4; o > 0; o >>= 1) {
+            Part<ZT> y; y.v = shfl_xor_t<ZT>(acc.v, o); y.has = __shfl_xor_sync(0xffffffffu, acc.has, o);
             acc = part_join<ZT>(ADD, acc, y);
         }
+        if (ok && sub == 0) { static_cast<ZT *>(p.tval)[f.row] = acc.v; if (SPARSE) p.tpres[f.row] = (uint8_t)acc.has; }
+        return;
     }
+    const int64_t i = ((int64_t)blockIdx.x - long_ctas) * 256 + threadIdx.x;
+    if (i >= p.fix_short) return;
+    const uint4 w = __ldg(reinterpret_cast<const uint4 *>(p.fix + p.fix_long + i));
+    const uint32_t run = w.x, row = w.y, n = w.z - w.x;                 // heads run+1 .. run+n, n <= FIX_LANES
+    Part<ZT> l[FIX_LANES];                                               // l[s]: what lane s of the 8-lane form holds
+#pragma unroll
+    for (int s = 0; s < (int)FIX_LANES; ++s) {
+        l[s].has = (uint32_t)s < n ? (SPARSE ? (int)p.head_has[run + 1 + s] : 1) : 0;
+        l[s].v = (uint32_t)s < n ? head[run + 1 + s] : (ZT)0;
+    }
+    const Part<ZT> tail{static_cast<const ZT *>(p.tail_val)[run], SPARSE ? (int)p.tail_has[run] : 1};
+    l[0] = part_join<ZT>(ADD, tail, l[0]);
 #pragma unroll
     for (int o = 4; o > 0; o >>= 1) {
-        Part<ZT> y; y.v = shfl_xor_t<ZT>(acc.v, o); y.has = __shfl_xor_sync(0xffffffffu, acc.has, o);
-        acc = part_join<ZT>(ADD, acc, y);
+#pragma unroll
+        for (int s = 0; s < o; ++s) l[s] = part_join<ZT>(ADD, l[s], l[s + o]);
     }
-    if (r >= 0 && sub == 0) { static_cast<ZT *>(p.tval)[r] = acc.v; if (SPARSE) p.tpres[r] = (uint8_t)acc.has; }
+    static_cast<ZT *>(p.tval)[row] = l[0].v;
+    if (SPARSE) p.tpres[row] = (uint8_t)l[0].has;
+}
+
+// nnz > 0: the first row start makes at least one item
+template <typename ZT, int ADD, bool SPARSE> static void spmv_run_fixup(const RunArgs &a) {
+    const int64_t ctas = ceil_div(a.fix_long * FIX_LANES, 256) + ceil_div(a.fix_short, 256);
+    launch_pdl(spmv_run_fixup_kernel<ZT, ADD, SPARSE>, (unsigned)ctas, 256, 0, a); GB_LAUNCHED();
 }
 
 // shared memory the hot-table kernel can use for its table, after the warp stages and barriers
@@ -346,22 +427,22 @@ static void spmv_run_launch(const RunArgs &a, const Hot2Args *hot, size_t table_
                 auto kernel = spmv_run_hot2_kernel<XT, ZT, ADD, MUL, true>;
                 static size_t set_for = 0;
                 if (set_for != smem) { cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem); set_for = smem; }
-                kernel<<<ctas, HOT2_WARPS * 32, smem, G.stream>>>(a, h); GB_LAUNCHED();
+                launch_pdl(kernel, (unsigned)ctas, HOT2_WARPS * 32, smem, a, h); GB_LAUNCHED();
             } else {
                 auto kernel = spmv_run_hot2_kernel<XT, ZT, ADD, MUL, false>;
                 static size_t set_for = 0;
                 if (set_for != smem) { cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem); set_for = smem; }
-                kernel<<<ctas, HOT2_WARPS * 32, smem, G.stream>>>(a, h); GB_LAUNCHED();
+                launch_pdl(kernel, (unsigned)ctas, HOT2_WARPS * 32, smem, a, h); GB_LAUNCHED();
             }
-            spmv_run_fixup_kernel<ZT, ADD, false><<<(unsigned)ceil_div(a.nruns * 8, 256), 256, 0, G.stream>>>(a); GB_LAUNCHED();
+            spmv_run_fixup<ZT, ADD, false>(a);
             return;
         }
     }
     if (a.upres) {
         spmv_run_kernel<XT, ZT, ADD, MUL, true><<<(unsigned)ceil_div(a.nruns, 8), 256, 0, G.stream>>>(a); GB_LAUNCHED();
-        spmv_run_fixup_kernel<ZT, ADD, true><<<(unsigned)ceil_div(a.nruns * 8, 256), 256, 0, G.stream>>>(a); GB_LAUNCHED();
+        spmv_run_fixup<ZT, ADD, true>(a);
         return;
     }
     spmv_run_kernel<XT, ZT, ADD, MUL, false><<<(unsigned)ceil_div(a.nruns, 8), 256, 0, G.stream>>>(a); GB_LAUNCHED();
-    spmv_run_fixup_kernel<ZT, ADD, false><<<(unsigned)ceil_div(a.nruns * 8, 256), 256, 0, G.stream>>>(a); GB_LAUNCHED();
+    spmv_run_fixup<ZT, ADD, false>(a);
 }
